@@ -6,6 +6,7 @@
     python bench.py --impl reference ...        # the reference's arithmetic (oracle port) on the host cores
     python bench.py --impl library ...          # the same module graph under stock PyTorch eager (autocast, channels_last,
                                                 # cuDNN / cuBLAS, torch DDP over NCCL): the bar SURVEY.md 8(d) names
+    python bench.py --dump-outputs DIR ...      # also write what the last timed step computed as DIR/<name>.npy
 
 One "step" = one full train iteration of the reference's hot loop (dfd/runners/train.py:621-637) on a synthetic
 batch: forward, 2-class CE (sigmoid-BCE) loss + top-1, zero_grad, backward, [gradient all-reduce], SGD-nesterov
@@ -52,6 +53,31 @@ def load_peaks():
         d = json.load(open(p))
         return dict(hbm_gbs=d["hbm_gbs"], tf_burst=d["bf16_tflops"], tf_sustained=d["bf16_tflops_sustained"], source="measured")
     return dict(hbm_gbs=6650.0, tf_burst=1590.0, tf_sustained=1400.0, source="fallback")
+
+
+DUMP_BYTES = 60 << 20      # all dumped arrays together, leaving room for the .npy headers under 64 MB
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Write each tensor as out_dir/<name>.npy (float64 stays float64, everything else becomes float32).
+
+    The arrays are taken smallest first and each may use an equal share of what is left of `budget`.  One larger than its
+    share is replaced by a sample of its flattened elements at positions drawn from a fixed seed, so the same array size
+    always gives the same positions and two builds can be compared element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = budget
+    for i, (name, t) in enumerate(items):
+        t = t.detach().cpu()
+        a = (t.double() if t.dtype == torch.float64 else t.float()).numpy()
+        share = left // (len(items) - i)
+        if a.nbytes > share:
+            idx = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
 
 
 class ClockSampler(threading.Thread):
@@ -284,6 +310,14 @@ def run_native(args):
         t = torch.tensor([ms], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the step receives after the last timed step: loss, correct count, logits, the reference-layout
+        # state dict (updated weights, running statistics) and the gradients, flattened in parameter order
+        sd = tr.state_dict()
+        dump_outputs(args.dump_outputs, dict(
+            loss=e.loss.reshape(1), correct=e.correct.reshape(1), logits=e.logits,
+            state=torch.cat([v.reshape(-1).float() for v in sd.values()]),
+            grads=torch.cat([e.grad_view(n).reshape(-1) for n in e.param_names])))
 
     # ---- end to end through the public API with HOST buffers (H2D of the batch + D2H of the loss every step) ----
     # the batch is what the reference's fast_collate hands its prefetcher: uint8 NCHW in pinned host memory
@@ -621,7 +655,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=4)
     ap.add_argument("--cpu-world", type=int, default=1, help="--impl reference: also time N gloo ranks on the host cores")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl native: write the outputs of the last timed step as DIR/<name>.npy (64 MB at most)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs is only implemented for --impl native")
     if args.impl == "reference":
         run_reference(args)
     elif args.impl == "library":

@@ -76,6 +76,27 @@ def test_bench_native_arm_does_not_touch_the_oracle():
     assert not re.search(r"(from|import)\s+oracle", native)
 
 
+def test_bench_dump_outputs_stays_in_budget_and_samples_the_same_positions(tmp_path):
+    """bench.py --dump-outputs: small arrays are written whole, a large one as a fixed-seed sample, all of them within the
+    byte budget; a second dump of the same arrays is identical."""
+    import numpy as np
+    import torch
+    import bench
+    g = torch.Generator().manual_seed(0)
+    arrays = dict(loss=torch.tensor([0.5]), logits=torch.randn(8, 2, generator=g), state=torch.randn(5000, generator=g),
+                  grads=torch.randn(3000, generator=g, dtype=torch.float64))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, budget=16384)
+    got = {f[:-4]: np.load(str(tmp_path / "a" / f)) for f in os.listdir(str(tmp_path / "a"))}
+    assert set(got) == set(arrays)
+    assert sum(os.path.getsize(str(tmp_path / "a" / (n + ".npy"))) - 128 for n in got) <= 16384
+    assert got["logits"].dtype == np.float32 and np.array_equal(got["logits"], arrays["logits"].numpy())
+    assert got["grads"].dtype == np.float64 and got["state"].dtype == np.float32
+    assert 0 < got["state"].size < 5000 and np.isin(got["state"], arrays["state"].numpy()).all()
+    for n in got:
+        assert np.array_equal(got[n], np.load(str(tmp_path / "b" / (n + ".npy")))), n
+
+
 def test_row_pack_rule():
     """small-K pointwise convs are read `pack` rows at a time; pack must divide M and only applies below 64 channels"""
     from deepfake_detection_b200.engine import Engine
