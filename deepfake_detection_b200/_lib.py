@@ -53,6 +53,7 @@ SIGNATURES = {
     "dfd_se_fc_wgrad": "pppp" "pppp" "iii" "p",
     "dfd_pool_se": "pppp" "ppppp" "ili" "iii" "i" "p",
     "dfd_se_bwd_chain": "ppppp" "ppppp" "pppp" "ili" "ii" "p",
+    "dfd_head_max_classes": "",
     "dfd_head_fwd": "pppp" "iii" "pp" "ff" "pppp" "p",
     "dfd_head_bwd": "pppppp" "iii" "p",
     "dfd_sgd_step": "ppp" "l" "fffi" "f" "ppp" "i" "p" "p",
@@ -107,6 +108,7 @@ class _Lib:
         if self.cdll.dfd_abi_version() != 1:
             raise NativeError("libdfd_b200.so ABI version mismatch")
         self.stat_slots = self.cdll.dfd_stat_slots()
+        self.head_kmax = self.cdll.dfd_head_max_classes()      # largest num_classes the classifier kernels take
 
     def last_error(self):
         return self.cdll.dfd_last_error().decode("utf-8", "replace")

@@ -1,10 +1,11 @@
-// Small per-image kernels (squeeze-excite FCs, classifier + sigmoid-BCE loss) and the flat-arena
+// Small per-image kernels (squeeze-excite FCs, classifier + cross-entropy loss) and the flat-arena
 // optimizer / weight-preparation kernels.
 //
 // Reference semantics restated here:
 //   SqueezeExcite.forward         dfd/timm/models/efficientnet_blocks.py:104-110  (FC+bias, Swish, FC+bias, sigmoid)
 //   classifier + loss             dfd/timm/models/efficientnet.py:348, dfd/timm/loss/cross_entropy.py:20-36,
-//                                 nn.CrossEntropyLoss (dfd/runners/train.py:509-520); 2-class CE == sigmoid-BCE on z1-z0
+//                                 nn.CrossEntropyLoss (dfd/runners/train.py:509-520); 2-class CE == sigmoid-BCE on z1-z0,
+//                                 any other class count: softmax-CE (head_loss_kernel)
 //   accuracy                      dfd/timm/utils.py:170-186
 //   SGD nesterov                  torch.optim.SGD as configured by dfd/timm/optim/optim_factory.py:48-50
 //   Adam / AdamW                  optim_factory.py:51-56, dfd/timm/optim/adamw.py:55-117
@@ -252,7 +253,7 @@ __global__ void se_fc_wgrad_kernel(const float* __restrict__ d_e, const float* _
 }
 
 // ---------------------------------------------------------------------------------------------
-// classifier: logits[n,k] = W[k,:] . pooled[n,:] + b[k]   (one CTA per image, one warp per class round-robin)
+// 2-class classifier: logits[n,k] = W[k,:] . pooled[n,:] + b[k]   (one CTA per image, one warp per class round-robin)
 // fused 2-class loss (sigmoid-BCE on d = z1 - z0 == softmax-CE), top-1, and dL/dlogits.
 // target: int64 hard labels (tgt_i) or float soft targets [N,2] (tgt_f).
 // ---------------------------------------------------------------------------------------------
@@ -347,6 +348,213 @@ __global__ void head_wgrad_kernel(const float* __restrict__ dlogits, const float
     }
     dW[idx] += s;
     if (f == 0) db[k] += sb;
+}
+
+// ---------------------------------------------------------------------------------------------
+// K-class head (every K != 2 up to HEAD_KMAX): softmax cross-entropy with the reference's three target encodings.
+// The three products of the classifier run through one fp32 tile kernel; the loss / top-1 / dL/dlogits run one CTA per
+// image row.  Every output is a single fixed-order sum (no split partials, no atomics), so results are bit-reproducible.
+// ---------------------------------------------------------------------------------------------
+constexpr int HEAD_KMAX = 4096;
+constexpr int HG_BK = 16;            // contraction depth of one shared-memory stage
+constexpr int HL_THREADS = 256;
+
+// C[m, c] (+)= sum_r A(m, r) B(r, c) (+ bias[c]).  A(m, r) = A[m*lda + r] if A_RC (contraction index contiguous), else
+// A[r*lda + m]; B(r, c) = B[c*ldb + r] if B_RC, else B[r*ldb + c].  A BM x BN tile per CTA, 4 x 4 outputs per thread; the
+// next HG_BK-deep stage is loaded into registers while the current one is multiplied out of shared memory.  Every output
+// accumulates r = 0, 1, ..., R-1 in order whatever the tile shape, so the launcher's tile choice never changes a bit.
+template <int BM, int BN, bool A_RC, bool B_RC>
+__global__ void __launch_bounds__((BM / 4) * (BN / 4))
+head_gemm_kernel(const float* __restrict__ A, int lda, const float* __restrict__ B, int ldb, float* __restrict__ C, int ldc,
+                 const float* __restrict__ bias, int accumulate, int M, int Nc, int R) {
+    constexpr int NT = (BM / 4) * (BN / 4), LA = HG_BK * BM / NT, LB = HG_BK * BN / NT;
+    __shared__ __align__(16) float As[HG_BK][BM + 4];
+    __shared__ __align__(16) float Bs[HG_BK][BN + 4];
+    const int tid = threadIdx.x, tx = tid % (BN / 4), ty = tid / (BN / 4);
+    const int m0 = blockIdx.y * BM, c0 = blockIdx.x * BN;
+    float ra[LA], rb[LB];
+    // element e of a stage: the operand's contiguous index runs fastest across the threads (coalesced loads)
+    auto fetch = [&](int r0) {
+#pragma unroll
+        for (int i = 0; i < LA; i++) {
+            const int e = tid + i * NT;
+            const int r = A_RC ? e % HG_BK : e / BM, m = A_RC ? e / HG_BK : e % BM;
+            const int gm = m0 + m, gr = r0 + r;
+            ra[i] = (gm < M && gr < R) ? (A_RC ? A[(size_t)gm * lda + gr] : A[(size_t)gr * lda + gm]) : 0.f;
+        }
+#pragma unroll
+        for (int i = 0; i < LB; i++) {
+            const int e = tid + i * NT;
+            const int r = B_RC ? e % HG_BK : e / BN, c = B_RC ? e / HG_BK : e % BN;
+            const int gc = c0 + c, gr = r0 + r;
+            rb[i] = (gc < Nc && gr < R) ? (B_RC ? B[(size_t)gc * ldb + gr] : B[(size_t)gr * ldb + gc]) : 0.f;
+        }
+    };
+    float acc[4][4];
+#pragma unroll
+    for (int i = 0; i < 4; i++)
+#pragma unroll
+        for (int j = 0; j < 4; j++) acc[i][j] = 0.f;
+    fetch(0);
+    for (int r0 = 0; r0 < R; r0 += HG_BK) {
+#pragma unroll
+        for (int i = 0; i < LA; i++) {
+            const int e = tid + i * NT;
+            As[A_RC ? e % HG_BK : e / BM][A_RC ? e / HG_BK : e % BM] = ra[i];
+        }
+#pragma unroll
+        for (int i = 0; i < LB; i++) {
+            const int e = tid + i * NT;
+            Bs[B_RC ? e % HG_BK : e / BN][B_RC ? e / HG_BK : e % BN] = rb[i];
+        }
+        __syncthreads();
+        if (r0 + HG_BK < R) fetch(r0 + HG_BK);
+#pragma unroll
+        for (int r = 0; r < HG_BK; r++) {
+            const float4 a = *reinterpret_cast<const float4*>(&As[r][ty * 4]);
+            const float4 b = *reinterpret_cast<const float4*>(&Bs[r][tx * 4]);
+            const float av[4] = {a.x, a.y, a.z, a.w}, bv[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+            for (int i = 0; i < 4; i++)
+#pragma unroll
+                for (int j = 0; j < 4; j++) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const int m = m0 + ty * 4 + i;
+        if (m >= M) continue;
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int c = c0 + tx * 4 + j;
+            if (c >= Nc) continue;
+            float* out = C + (size_t)m * ldc + c;
+            float v = acc[i][j];
+            if (bias) v += bias[c];
+            *out = accumulate ? *out + v : v;
+        }
+    }
+}
+
+// block-wide sum in a fixed order (butterfly within warps, warp partials in warp order); every thread gets the result
+__device__ __forceinline__ float block_sum_ordered(float v, float* red) {
+    v = warp_sum(v);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    __syncthreads();
+    if (lane == 0) red[warp] = v;
+    __syncthreads();
+    float s = 0.f;
+    for (int w = 0; w < (int)(blockDim.x >> 5); w++) s += red[w];
+    return s;
+}
+
+// block-wide (max, first index of the max); every thread gets the result
+__device__ __forceinline__ void argmax_merge(float& v, int& i, float ov, int oi) {
+    if (ov > v || (ov == v && oi < i)) { v = ov; i = oi; }
+}
+__device__ __forceinline__ void block_argmax(float& v, int& i, float* redv, int* redi) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) argmax_merge(v, i, __shfl_xor_sync(0xffffffffu, v, o), __shfl_xor_sync(0xffffffffu, i, o));
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    __syncthreads();
+    if (lane == 0) { redv[warp] = v; redi[warp] = i; }
+    __syncthreads();
+    v = redv[0]; i = redi[0];
+    for (int w = 1; w < (int)(blockDim.x >> 5); w++) argmax_merge(v, i, redv[w], redi[w]);
+}
+
+// one CTA per image row of logits [N, K]:
+//   t_k = smoothing/K + (1 - smoothing)[k == y]  (hard label y, clamped into the row)  or  t = tgt_f[n, :] (soft),
+//   loss_n = sum_k t_k (lse - z_k),  dlogits = (sum_k t_k * softmax(z) - t) / N * loss_scale,
+//   pred = first index of the row max, label = y or the first argmax of the soft target row.
+// The per-image loss / hit land in fixed slots and the last CTA adds them in image order (as head_fwd_kernel does).
+__global__ void __launch_bounds__(HL_THREADS)
+head_loss_kernel(const float* __restrict__ logits, int K, const long long* __restrict__ tgt_i,
+                 const float* __restrict__ tgt_f, float smoothing, float inv_n, float loss_scale,
+                 const float* __restrict__ loss_scale_dev, float* __restrict__ loss_acc, float* __restrict__ correct_acc,
+                 float* __restrict__ dlogits) {
+    __shared__ float redv[32];
+    __shared__ int redi[32];
+    const int n = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
+    const float* z = logits + (size_t)n * K;
+    const float* t = tgt_f ? tgt_f + (size_t)n * K : nullptr;
+    float zmax = -INFINITY;
+    int pred = K;
+    for (int k = tid; k < K; k += nt) {
+        const float v = z[k];
+        if (pred == K || v > zmax) { zmax = v; pred = k; }
+    }
+    block_argmax(zmax, pred, redv, redi);
+    int y = 0;
+    if (!t) {
+        const long long yl = tgt_i[n];
+        y = yl < 0 ? 0 : (yl >= K ? K - 1 : (int)yl);
+    }
+    const float off = t ? 0.f : smoothing / (float)K, on = 1.f - smoothing + off;
+    float se = 0.f, st = 0.f, tmax = -INFINITY;
+    int lab = t ? K : y;
+    for (int k = tid; k < K; k += nt) {
+        se += expf(z[k] - zmax);
+        if (t) {
+            const float tk = t[k];
+            st += tk;
+            if (lab == K || tk > tmax) { tmax = tk; lab = k; }
+        }
+    }
+    se = block_sum_ordered(se, redv);
+    if (t) {
+        st = block_sum_ordered(st, redv);
+        block_argmax(tmax, lab, redv, redi);
+    } else {
+        st = 1.f;          // sum_k t_k is exactly 1 for a smoothed one-hot target
+    }
+    const float lse = zmax + logf(se);
+    const float ls = (loss_scale_dev ? loss_scale * *loss_scale_dev : loss_scale) * inv_n;
+    float loss = 0.f;
+    for (int k = tid; k < K; k += nt) {
+        const float v = z[k];
+        const float tk = t ? t[k] : (k == y ? on : off);
+        loss = fmaf(tk, lse - v, loss);
+        if (dlogits) dlogits[(size_t)n * K + k] = (st * (expf(v - zmax) / se) - tk) * ls;
+    }
+    loss = block_sum_ordered(loss, redv);
+    if (tid == 0) {
+        g_small_ws[n] = loss * inv_n;
+        g_small_ws[gridDim.x + n] = pred == lab ? 1.f : 0.f;
+    }
+    if (!ticket_last(g_small_tk, gridDim.x)) return;
+    if (tid == 0) {
+        float l = 0.f, c = 0.f;
+        for (int i = 0; i < (int)gridDim.x; i++) { l += __ldcg(g_small_ws + i); c += __ldcg(g_small_ws + gridDim.x + i); }
+        *loss_acc += l;
+        *correct_acc += c;
+    }
+}
+
+// db[k] += sum_n dlogits[n, k], images in order
+__global__ void head_bias_grad_kernel(const float* __restrict__ dlogits, float* __restrict__ db, int N, int K) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= K) return;
+    float s = 0.f;
+#pragma unroll 8
+    for (int n = 0; n < N; n++) s += dlogits[(size_t)n * K + k];
+    db[k] += s;
+}
+
+// the tile shape: the largest of 64 x 64 / 32 x 64 / 32 x 32 that still gives the 148 SMs work (more, smaller CTAs for the
+// small products of the head); results do not depend on it
+template <bool A_RC, bool B_RC>
+static int head_gemm(const float* A, int lda, const float* B, int ldb, float* C, int ldc, const float* bias, int accumulate,
+                     int M, int Nc, int R, cudaStream_t st) {
+    if ((long long)cdiv(M, 64) * cdiv(Nc, 64) >= 2 * 148)
+        head_gemm_kernel<64, 64, A_RC, B_RC><<<dim3(cdiv(Nc, 64), cdiv(M, 64)), 256, 0, st>>>(A, lda, B, ldb, C, ldc, bias, accumulate, M, Nc, R);
+    else if ((long long)cdiv(M, 32) * cdiv(Nc, 64) >= 148)
+        head_gemm_kernel<32, 64, A_RC, B_RC><<<dim3(cdiv(Nc, 64), cdiv(M, 32)), 128, 0, st>>>(A, lda, B, ldb, C, ldc, bias, accumulate, M, Nc, R);
+    else
+        head_gemm_kernel<32, 32, A_RC, B_RC><<<dim3(cdiv(Nc, 32), cdiv(M, 32)), 64, 0, st>>>(A, lda, B, ldb, C, ldc, bias, accumulate, M, Nc, R);
+    DFD_LAUNCH_CHECK();
+    return DFD_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -616,15 +824,27 @@ int dfd_se_fc_wgrad(const float* d_e, const float* r, const float* d_rpre, const
     return DFD_OK;
 }
 
+int dfd_head_max_classes(void) { return HEAD_KMAX; }
+
 int dfd_head_fwd(const float* pooled, const float* W, const float* b, float* logits, int N, int F, int K,
                  const long long* tgt_i, const float* tgt_f, float smoothing, float loss_scale,
                  const float* loss_scale_dev, float* loss_acc, float* correct_acc, float* dlogits, void* stream) {
-    if (N <= 0 || F <= 0 || K <= 0 || K > 32) return dfd_set_error(DFD_ERR_ARG, "dfd_head_fwd: sizes");
-    if (loss_acc && K != 2) return dfd_set_error(DFD_ERR_UNSUPPORTED, "dfd_head_fwd: fused sigmoid-BCE needs num_classes == 2");
+    if (N <= 0 || F <= 0 || K <= 0) return dfd_set_error(DFD_ERR_ARG, "dfd_head_fwd: sizes");
+    if (K > HEAD_KMAX) return dfd_set_error(DFD_ERR_UNSUPPORTED, "dfd_head_fwd: num_classes exceeds DFD_HEAD_KMAX (4096)");
+    if (loss_acc && K < 2) return dfd_set_error(DFD_ERR_UNSUPPORTED, "dfd_head_fwd: a cross-entropy loss needs num_classes >= 2");
     if (loss_acc && !tgt_i && !tgt_f) return dfd_set_error(DFD_ERR_ARG, "dfd_head_fwd: loss without target");
     if (loss_acc && 2 * (long long)N > SMALL_WS_FLOATS) return dfd_set_error(DFD_ERR_UNSUPPORTED, "dfd_head_fwd: batch exceeds the reduction scratch");
-    head_fwd_kernel<<<N, 64, 0, (cudaStream_t)stream>>>(pooled, W, b, logits, F, K, tgt_i, tgt_f, smoothing,
-                                                         1.f / (float)N, loss_scale, loss_scale_dev, loss_acc, correct_acc, dlogits);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (K != 2) {
+        int rc = head_gemm<true, true>(pooled, F, W, F, logits, K, b, 0, N, K, F, st);               // logits = pooled W^T + b
+        if (rc || !loss_acc) return rc;
+        head_loss_kernel<<<N, HL_THREADS, 0, st>>>(logits, K, tgt_i, tgt_f, smoothing, 1.f / (float)N, loss_scale,
+                                                   loss_scale_dev, loss_acc, correct_acc, dlogits);
+        DFD_LAUNCH_CHECK();
+        return DFD_OK;
+    }
+    head_fwd_kernel<<<N, 64, 0, st>>>(pooled, W, b, logits, F, K, tgt_i, tgt_f, smoothing,
+                                      1.f / (float)N, loss_scale, loss_scale_dev, loss_acc, correct_acc, dlogits);
     DFD_LAUNCH_CHECK();
     return DFD_OK;
 }
@@ -632,7 +852,17 @@ int dfd_head_fwd(const float* pooled, const float* W, const float* b, float* log
 int dfd_head_bwd(const float* dlogits, const float* pooled, const float* W, float* dW, float* db, float* dpooled,
                  int N, int F, int K, void* stream) {
     if (N <= 0 || F <= 0 || K <= 0) return dfd_set_error(DFD_ERR_ARG, "dfd_head_bwd: sizes");
+    if (K > HEAD_KMAX) return dfd_set_error(DFD_ERR_UNSUPPORTED, "dfd_head_bwd: num_classes exceeds DFD_HEAD_KMAX (4096)");
     cudaStream_t st = (cudaStream_t)stream;
+    if (K != 2) {
+        int rc = head_gemm<true, false>(dlogits, K, W, F, dpooled, F, nullptr, 0, N, F, K, st);      // dpooled = dlogits W
+        if (rc) return rc;
+        rc = head_gemm<false, false>(dlogits, K, pooled, F, dW, F, nullptr, 1, K, F, N, st);         // dW += dlogits^T pooled
+        if (rc) return rc;
+        head_bias_grad_kernel<<<cdiv(K, 128), 128, 0, st>>>(dlogits, db, N, K);
+        DFD_LAUNCH_CHECK();
+        return DFD_OK;
+    }
     head_dgrad_kernel<<<cdiv((long long)N * F, 256), 256, 0, st>>>(dlogits, W, dpooled, N, F, K);
     DFD_LAUNCH_CHECK();
     head_wgrad_kernel<<<dim3(cdiv((long long)K * F, 128), N >= 64 ? 16 : (N >= 8 ? 4 : 1)), 128, 0, st>>>(dlogits, pooled, dW, db, N, F, K);

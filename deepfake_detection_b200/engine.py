@@ -11,6 +11,7 @@ PyTorch is used for device memory and streams only; there is no PyTorch compute 
 fallback: constructing an Engine without a CUDA device or without libdfd_b200.so raises.
 """
 import ctypes
+import numbers
 import os
 from collections import OrderedDict
 
@@ -25,6 +26,15 @@ POOL_CHUNKS = 8          # row chunks per image of the pooling kernels when the 
 
 def _ptr(t, off_elems=0):
     return t.data_ptr() + off_elems * t.element_size()
+
+
+def check_num_classes(num_classes):
+    """The classifier kernels take 1 <= num_classes <= DFD_HEAD_KMAX; refused here, before any plan or graph exists.
+    0 (timm's identity classifier, pooled features out) has no native path."""
+    kmax = _lib.lib().head_kmax
+    if not isinstance(num_classes, numbers.Integral) or not 1 <= num_classes <= kmax:
+        raise ValueError("num_classes=%r: the native classifier takes 1 <= num_classes <= %d (num_classes=0, the "
+                         "identity classifier, is not supported)" % (num_classes, kmax))
 
 
 class _BN:
@@ -45,6 +55,7 @@ class Engine:
             raise _lib.NativeError("deepfake_detection_b200.Engine needs a CUDA device (B200, sm_100a); "
                                    "there is no CPU path")
         self.L = _lib.lib()
+        check_num_classes(num_classes)
         self.spec = spec = get_spec(arch, num_classes=num_classes, in_chans=in_chans)
         self.cls_name = "classifier" if spec.family == "efficientnet" else "fc"
         self.device = torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
@@ -868,7 +879,7 @@ class Engine:
         return self.logits
 
     def head(self, with_loss, smoothing=0.0, loss_scale=1.0, soft=False, stream=None, loss_scale_dev=None):
-        """classifier (+ fused sigmoid-BCE loss, top-1 count and dL/dlogits when with_loss)."""
+        """classifier (+ fused softmax cross-entropy, top-1 count and dL/dlogits when with_loss; needs num_classes >= 2)."""
         st = stream if stream is not None else torch.cuda.current_stream().cuda_stream
         spec = self.spec
         pw = _ptr(self.params32, self.p_off[self.cls_name + ".weight"][0])

@@ -1,8 +1,9 @@
 """Train losses with the reference's names and semantics (dfd/timm/loss/cross_entropy.py:6-36).
 
-On `[N, 2]` logits these are a handful of tiny torch ops; when the runner is given one of these objects together with
-a NativeModel it uses the fused classifier + sigmoid-BCE kernel instead (`native_smoothing` / `native_soft` tell it
-which target encoding to use) — 2-class softmax-CE and sigmoid-BCE on z1 - z0 are the same function."""
+On `[N, K]` logits these are a handful of tiny torch ops; when the runner is given one of these objects together with
+a NativeModel it uses the fused classifier + softmax cross-entropy kernels instead (`native_smoothing` / `native_soft`
+tell it which target encoding to use), for any 2 <= K <= DFD_HEAD_KMAX. At K = 2 the kernel computes sigmoid-BCE on
+z1 - z0, which is the same function as 2-class softmax-CE."""
 import torch
 import torch.nn as nn
 import torch.nn.functional as F

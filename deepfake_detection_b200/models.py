@@ -19,7 +19,7 @@ import torch.nn as nn
 
 from . import _lib
 from .arch import SUPPORTED_ARCHS, get_spec, state_entries
-from .engine import Engine
+from .engine import Engine, check_num_classes
 
 _DEFAULT_CFG = dict(num_classes=1000, pool_size=(7, 7), crop_pct=0.875, interpolation="bicubic",
                     mean=(0.485, 0.456, 0.406), std=(0.229, 0.224, 0.225))
@@ -106,6 +106,7 @@ class NativeModel(nn.Module):
         if bn_tf:       # efficientnet_blocks.py:13-30
             bn_momentum = 1 - 0.99 if bn_momentum is None else bn_momentum
             bn_eps = 1e-3 if bn_eps is None else bn_eps
+        check_num_classes(num_classes)
         self.arch = arch
         self.num_classes = num_classes
         self.in_chans = in_chans

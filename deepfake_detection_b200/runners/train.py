@@ -13,7 +13,7 @@ The reported numbers are identical.
 
 Two step flavours:
   * fused   : model is a NativeModel, loss_fn one of deepfake_detection_b200.loss.* and optimizer an ArenaOptimizer
-              -> one Trainer step (forward, sigmoid-BCE head, backward, [all-reduce], update), CUDA-graph replayed;
+              -> one Trainer step (forward, cross-entropy head, backward, [all-reduce], update), CUDA-graph replayed;
   * protocol: anything else that follows the reference's object protocol (model(input), loss_fn(out, target),
               loss.backward(), optimizer.step()) — the NativeModel autograd bridge makes this work unchanged.
 """

@@ -223,7 +223,17 @@ int dfd_se_bwd_chain(const void* da, const void* y, const float* scale, const fl
 
 /* ---- classifier + loss + accuracy: nn.Linear (efficientnet.py:348, resnet.py:467), LabelSmoothing /
  *      SoftTarget / nn.CrossEntropyLoss (loss/cross_entropy.py:20-36, train.py:509-520), accuracy
- *      (utils.py:170-186).  2-class softmax-CE is computed as sigmoid-BCE on z1 - z0 (exactly equal). ----- */
+ *      (utils.py:170-186).  Any class count 1 <= K <= DFD_HEAD_KMAX; the loss needs K >= 2.
+ *   K == 2: one CTA per image, softmax-CE computed as sigmoid-BCE on z1 - z0 (exactly equal).
+ *   K != 2: fp32 shared-memory tile products for the logits, dpooled and dW, and one CTA per image for the softmax-CE
+ *           (lse = max + log sum exp(z - max); targets t_k = smoothing/K + (1 - smoothing)[k == y], or the soft row),
+ *           top-1 (first index of the row max; the label of a soft row is its first argmax) and dL/dlogits.
+ *   Every output is one sum in a fixed order (no atomics, no split partials), so results are bit-reproducible. Logits-only
+ *   calls with K = 3..32 sum over F in a different order than before DFD_HEAD_KMAX existed (last-bit differences).
+ *   Labels are clamped into [0, K-1]. K > DFD_HEAD_KMAX, or a loss with K < 2, returns DFD_ERR_UNSUPPORTED.
+ *   dfd_head_bwd: dpooled = dlogits W (overwritten); dW += dlogits^T pooled, db += sum_n dlogits (accumulated). ----- */
+#define DFD_HEAD_KMAX 4096
+int dfd_head_max_classes(void);
 int dfd_head_fwd(const float* pooled, const float* W, const float* b, float* logits, int N, int F, int K,
                  const long long* target_i64, const float* target_soft, float smoothing, float loss_scale,
                  const float* loss_scale_dev, float* loss_acc, float* correct_acc, float* dlogits, void* stream);
